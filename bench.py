@@ -22,6 +22,9 @@ committed oracle results.
 
 --impl reference : the C restatement of the reference CPU path (oracle/cref, all usable host threads)
 on the 2^20-leaf prefix of the same leaf stream (the Rust reference cannot be built in this image).
+
+--dump-outputs DIR : after the timed steps, write what the last one returned (root, leaf digests, inner
+nodes) to DIR/*.npy (dump_tree), so that two builds can be compared output for output on the same inputs.
 """
 from __future__ import annotations
 
@@ -65,6 +68,29 @@ def goldens():
 def u64_list(t):
     """4-limb digest tensor/array -> list of unsigned limbs (JSON-able, comparable with the golden file)."""
     return [int(x) & MASK64 for x in (t.reshape(-1).tolist())]
+
+
+DUMP_SAMPLE = 1 << 18           # digests per sampled array: 16 MB each as float64 words, about 36 MB per dump in all
+DUMP_SEED = 0xB20000D0
+
+
+def dump_tree(tree, out_dir):
+    """Writes the arrays one tree build hands its caller: root.npy (8,), and leaf_nodes.npy / non_leaf_nodes.npy (k, 8) at a
+    fixed, seeded sample of k <= DUMP_SAMPLE indices (ascending; heap order for the inner nodes), stored in *_index.npy.
+    A digest is 4 little-endian 64-bit Montgomery limbs; each row holds its eight 32-bit words as float64, which is exact."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+
+    def words(t):
+        return t.contiguous().cpu().numpy().view(np.uint32).astype(np.float64)
+
+    np.save(os.path.join(out_dir, "root.npy"), words(tree.root.reshape(1, -1))[0])
+    rng = np.random.default_rng(DUMP_SEED)
+    for name, a in (("leaf_nodes", tree.local_leaf_nodes), ("non_leaf_nodes", tree.local_nodes)):
+        idx = np.sort(rng.choice(a.shape[0], min(DUMP_SAMPLE, a.shape[0]), replace=False))
+        np.save(os.path.join(out_dir, f"{name}.npy"), words(a[torch.from_numpy(idx).to(a.device)]))
+        np.save(os.path.join(out_dir, f"{name}_index.npy"), idx.astype(np.float64))
 
 
 # --------------------------------------------------------------------------------- clocks sampler
@@ -268,6 +294,8 @@ def run_b200(args):
     if world != args.gpus:
         if world == 1 and args.gpus > 1:
             raise SystemExit("launch with torchrun --nproc-per-node N for --gpus N > 1")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes the outputs of a one-GPU build: use it with --gpus 1")
     torch.cuda.set_device(local_rank)
     dev = torch.device("cuda", local_rank)
     if world > 1:
@@ -334,6 +362,8 @@ def run_b200(args):
         root = tree.root.clone()
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dump_tree(tree, args.dump_outputs)
     t = torch.tensor([sum(times)], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -682,7 +712,13 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default=DEFAULT_WORKLOAD, choices=list(WORKLOADS))
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's root, leaf digests and inner nodes to DIR/*.npy (see dump_tree)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU build (--impl b200)")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,5 +1,6 @@
 """bench.py's CPU arm (`--impl reference`: the C restatement of the reference path on the host cores) runs without a GPU
-and prints the contract's JSON line; under torchrun only rank 0 prints."""
+and prints the contract's JSON line; under torchrun only rank 0 prints.  Also the file format of --dump-outputs and the
+argument checks."""
 import json
 import os
 import subprocess
@@ -32,3 +33,39 @@ def test_reference_arm_prints_one_contract_line():
 
 def test_reference_arm_other_ranks_stay_silent():
     assert _run({"RANK": "1", "WORLD_SIZE": "2", "LOCAL_RANK": "1"}) == ""
+
+
+def test_dump_outputs_are_exact_float_images_of_a_fixed_sample(tmp_path):
+    """--dump-outputs (bench.dump_tree): float64 32-bit words that give back the limbs exactly, at the same indices every run."""
+    import types
+
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    n = 3 * bench.DUMP_SAMPLE // 2
+    g = torch.Generator().manual_seed(5)
+    leaf = torch.randint(-2**62, 2**62, (n, 4), dtype=torch.int64, generator=g)
+    nodes = torch.randint(-2**62, 2**62, (n - 1, 4), dtype=torch.int64, generator=g)
+    tree = types.SimpleNamespace(root=nodes[0], local_leaf_nodes=leaf, local_nodes=nodes)
+    for d in ("a", "b"):
+        bench.dump_tree(tree, str(tmp_path / d))
+
+    def limbs(w):
+        w = w.astype(np.uint64)
+        return w[..., 0::2] | (w[..., 1::2] << np.uint64(32))
+
+    assert np.array_equal(limbs(np.load(tmp_path / "a" / "root.npy")), nodes[0].numpy().view(np.uint64))
+    total = 0
+    for name, src in (("leaf_nodes", leaf), ("non_leaf_nodes", nodes)):
+        words, idx = (np.load(tmp_path / "a" / f"{name}{s}.npy") for s in ("", "_index"))
+        assert words.dtype == idx.dtype == np.float64 and words.shape == (bench.DUMP_SAMPLE, 8)
+        assert np.array_equal(limbs(words), src.numpy().view(np.uint64)[idx.astype(np.int64)])
+        assert np.array_equal(words, np.load(tmp_path / "b" / f"{name}.npy"))
+        total += words.nbytes + idx.nbytes
+    assert total <= 64 << 20
+
+
+def test_steps_below_one_are_rejected():
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True, cwd=ROOT, timeout=120)
+    assert r.returncode != 0 and "--steps" in r.stderr
