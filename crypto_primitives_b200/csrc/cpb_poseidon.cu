@@ -100,15 +100,6 @@ CPB_POS_EXTERN_TEAM(Bls12_377_Fr)
 
 namespace {
 
-PoseidonDev to_dev(const host::PoseidonSchedule& S) {
-    PoseidonDev D;
-    D.t = S.t; D.rate = S.rate; D.cap = S.capacity; D.rf = S.rf; D.rp = S.rp; D.sparse = S.sparse; D.alpha = S.alpha;
-    D.off_c = S.off_c; D.off_m = S.off_m; D.off_mpre = S.off_mpre; D.off_cp0 = S.off_cp0; D.off_pc = S.off_pc;
-    D.off_sp = S.off_sp; D.off_arkp = S.off_arkp; D.off_mod = S.off_mod; D.off_sc0 = S.off_sc0; D.n_elems = S.n_elems; D.zero = 0;
-    return D;
-}
-
-
 #define CPB_CASE_T(F, T, M, ...) case T: return M<F, T>(__VA_ARGS__);
 #define CPB_FOR_T(F, M, ...)                                                                                   \
     switch (c->dev.t) {                                                                                        \
@@ -546,7 +537,7 @@ cpb_status cpb_poseidon_ctx_create(int field_id, int rate, int capacity, int ful
     c->device = device;
     c->sms = sm_count(device);
     c->sched = host::derive_schedule(F, P, true);
-    c->dev = to_dev(c->sched);
+    c->dev = host::make_dev(c->sched);
     size_t bytes = c->sched.consts.size() * 8;
     if (bytes > 200 * 1024) { delete c; return fail(CPB_UNSUPPORTED, "round schedule (%zu B) exceeds shared memory", bytes); }
     cudaError_t e = cudaMalloc(&c->d_consts, bytes);

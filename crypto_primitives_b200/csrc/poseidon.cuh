@@ -21,6 +21,8 @@ struct PoseidonDev {
     // warp-uniform address are promoted to uniform registers, and a multiply-add with a
     // uniform-register factor is emitted as IMAD.X + IMAD.HI.U32.X instead of one IMAD.WIDE.U32.X.
     int zero;
+    // Lane-0 recurrence of the partial rounds (host::derive_recurrence); off unless the schedule sets it.
+    int recur = 0, off_rc = 0, off_rk = 0, off_rr = 0;
 };
 
 template <class F, int T> CPB_HD void pos_add_vec(u32 (&s)[T][8], const u32* c) {
@@ -81,6 +83,9 @@ template <class F> CPB_HD void pos_sbox(u32* x, u64 alpha, int top_bit, const u3
 #ifndef CPB_COL_UNROLL_MAX
 #define CPB_COL_UNROLL_MAX 4
 #endif
+#ifndef CPB_POS_RECUR
+#define CPB_POS_RECUR 1    // t = 3: partial rounds as the lane-0 recurrence when the schedule has one (pos_partial_recur)
+#endif
 
 // Sparse schedules only: the same permutation with the partial rounds in a loop of their own.  The two
 // halves of the full rounds share one body through a two-trip outer loop, so there is still a single
@@ -95,6 +100,62 @@ struct PermuteHint {
     int lane0_zero;        // != 0: state lane 0 is zero on entry
     unsigned need;         // bit i set: lane i of the result is read; everything else is dead
 };
+
+// The partial rounds of a t = 3 sparse schedule as the lane-0 recurrence of host::derive_recurrence.  Per round: the S-box, then
+// ONE five-term lazy dot over the history h = (y_k, y_k-1, y_k-2, x_k, x_k-1) -- 5 products and 1 Montgomery reduction, where the
+// sparse form's 3-term row and two reduced column products take 5 products and 3 reductions (BN254 Fr: 384 instead of 512 wide
+// multiply-adds).  Lanes 1, 2 are not carried through the rounds: the first two rounds read them from the history, and after the
+// last round two 4-term dots rebuild them, so the state leaves bit for bit as the sparse rounds leave it.
+// Ranges with `lazy` (BN254 Fr, alpha = 5; tests/test_poseidon_recurrence.py): x = d + c < 2p is kept unreduced except after the
+// last round, the S-box output y < 1.6p, so the history sums below 8.8p (EX = 4: nine canonical terms' worth) and the terms of the
+// rebuild below 6.2p (EX = 3).  Without it every value is canonical (EX = 0).
+template <class F, bool LZ> CPB_HD void pos_partial_recur(u32 (&s)[3][8], const PoseidonDev& P, const u32* cs, const u32* pm, bool lazy,
+                                                          int top_bit) {
+    constexpr int EXH = LZ ? 4 : 0, EXR = LZ ? 3 : 0;
+    const bool alpha_zero = P.alpha == 0;
+    u32 h[5][8];
+    fp_copy(h[1], s[1]);
+    fp_copy(h[2], s[2]);
+    fp_copy(h[3], s[0]);
+    fp_zero(h[4]);
+    const u32* row = cs + 8 * P.off_rc;      // rounds 0 and 1 have rows of their own, every later round uses the third
+    const u32* ck = cs + 8 * P.off_rk;
+#pragma unroll 1
+    for (int k = 0; k < P.rp; k++, ck += 8) {
+        fp_copy(h[0], h[3]);
+#if CPB_SBOX5
+        if (P.alpha == 5) {                   // straight-line x^5
+            u32 x2[8];
+            fp_sqr<F, LZ>(x2, h[0], pm);
+            fp_sqr<F, LZ>(x2, x2, pm);
+            fp_mul<F, LZ>(h[0], x2, h[0], pm);
+        } else
+#endif
+        if (alpha_zero) fp_one<F>(h[0]);
+        else pos_sbox<F>(h[0], P.alpha, top_bit, pm);
+        u32 d[8], c[8];
+        fp_dot<F, 5, EXH>(d, h, row, pm);
+        if (k < 2) row += 8 * 5;
+        ld_elem(c, ck);
+        fp_copy(h[2], h[1]);
+        fp_copy(h[1], h[0]);
+        fp_copy(h[4], h[3]);
+        if (lazy && k + 1 < P.rp) fp_add_noreduce(h[3], d, c);
+        else fp_add<F>(h[3], d, c);
+    }
+    // h[1..4] = (y_rp-1, y_rp-2, lane 0 after the last round, x_rp-1)
+    u32 g[4][8], c[8];
+#pragma unroll
+    for (int i = 0; i < 4; i++) fp_copy(g[i], h[i + 1]);
+    const u32* rr = cs + 8 * P.off_rr;
+    fp_copy(s[0], h[3]);
+    fp_dot<F, 4, EXR>(s[1], g, rr, pm);
+    ld_elem(c, rr + 8 * 8);
+    fp_add<F>(s[1], s[1], c);
+    fp_dot<F, 4, EXR>(s[2], g, rr + 8 * 4, pm);
+    ld_elem(c, rr + 8 * 9);
+    fp_add<F>(s[2], s[2], c);
+}
 
 template <class F, int T> CPB_HD void pos_permute_split(u32 (&s)[T][8], const PoseidonDev& P, const u32* cs, const u32* pm, const PermuteHint& H) {
     const int half = P.rf / 2;
@@ -127,6 +188,10 @@ template <class F, int T> CPB_HD void pos_permute_split(u32 (&s)[T][8], const Po
                 pos_rotl<T>(s);
             }
             const u32* rows = cs + 8 * ((phase == 0 && q == half - 1) ? P.off_mpre : P.off_m);
+            // (re)defined every round: the collector's old values are shifted through but never used, and without this they
+            // would count as live across the partial rounds
+#pragma unroll
+            for (int i = 0; i < T; i++) fp_zero(n[i]);
 #pragma unroll 1
             for (int i = 0; i < T; i++) {
                 u32 d[8];
@@ -141,6 +206,12 @@ template <class F, int T> CPB_HD void pos_permute_split(u32 (&s)[T][8], const Po
         }
         if (phase == 0 && P.rp > 0) {
             pos_add_vec<F, T>(s, cs + 8 * P.off_cp0);
+            if constexpr (T == 3 && CPB_POS_RECUR != 0) {
+                if (P.recur) {
+                    pos_partial_recur<F, LZ>(s, P, cs, pm, lazy, top_bit);
+                    continue;                 // (the end of phase 0)
+                }
+            }
             const u32* row = cs + 8 * P.off_sp;
             const u32* pc = cs + 8 * (P.off_pc + 1);
             // Partial rounds, lazy lane 0: lane 0 lives in [0, 2p) from the constant

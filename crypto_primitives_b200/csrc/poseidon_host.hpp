@@ -8,9 +8,13 @@
 //    dense t x t MDS in all RF+RP rounds; here the RP partial rounds use the equivalent
 //    sparse form (1 row + 1 column per round) with round constants folded so that only lane 0
 //    receives a constant.  The rewrite is exact field algebra, so outputs are bit-identical;
-//    when a required (t-1)x(t-1) minor is singular the schedule falls back to the dense form.
+//    when a required (t-1)x(t-1) minor is singular the schedule falls back to the dense form.  For t = 3 it adds the
+//    lane-0 recurrence of the partial rounds (derive_recurrence), which the one-hash-per-thread kernels run instead.
 #pragma once
+#include <algorithm>
+
 #include "hostfp.hpp"
+#include "poseidon.cuh"
 
 namespace cpb {
 namespace host {
@@ -132,6 +136,11 @@ struct PoseidonSchedule {
     int off_arkp = 0;  // rp x t   original partial-round constants                     (dense schedules only; empty when sparse)
     int off_mod = 0;   // 1        the modulus limbs (plain integer): the kernels load them from here into registers
     int off_sc0 = 0;   // 1        S(C[0][0]): lane 0 after the first S-box when it entered the permutation as zero (fresh sponge)
+    // Lane-0 recurrence of the partial rounds (t = 3 sparse schedules; see derive_recurrence).  recur == 0: not used, empty.
+    int recur = 0;
+    int off_rc = 0;    // 3 x 5    dot rows over the history (y_k, y_k-1, y_k-2, x_k, x_k-1): round 0, round 1, rounds >= 2
+    int off_rk = 0;    // rp       constant added to the dot of round k (gives x_k+1; for k = rp-1 the sparse lane 0 after the last round)
+    int off_rr = 0;    // 2x4 + 2  lanes 1, 2 after the last round from (y_rp-1, y_rp-2, lane 0, x_rp-1): two rows, two constants
     int n_elems = 0;
     std::vector<u64> consts;
 };
@@ -186,6 +195,100 @@ inline bool invert(const Field& F, FeVec A, int m, FeVec& out) {
         }
     }
     out = I;
+    return true;
+}
+
+// Affine forms over the variables of the partial-round linear system (the S-box outputs taken as free inputs):
+// entry 0 is the constant term, 1 and 2 lanes 1 and 2 on entry, 3 lane 0 on entry, 4 + k the S-box output y_k.
+inline FeVec form_var(const Field& F, int nv, int v) {
+    FeVec f((size_t)nv, F.zero());
+    if (v >= 0) f[(size_t)v] = F.one();
+    return f;
+}
+inline void form_axpy(const Field& F, FeVec& r, const Fe& c, const FeVec& a) {
+    for (size_t i = 0; i < r.size(); i++) r[i] = F.add(r[i], F.mul(c, a[i]));
+}
+// Coefficients c (free ones 0) with f - sum_i c_i g_i constant, and that constant k; false when there are none.
+inline bool solve_affine(const Field& F, const FeVec& f, const std::vector<FeVec>& g, FeVec& c, Fe& k) {
+    const int n = (int)g.size(), rows = (int)f.size() - 1;
+    std::vector<FeVec> A((size_t)rows, FeVec((size_t)n + 1));
+    for (int v = 0; v < rows; v++) {
+        for (int i = 0; i < n; i++) A[v][i] = g[i][(size_t)v + 1];
+        A[v][n] = f[(size_t)v + 1];
+    }
+    std::vector<int> pivcol;
+    int r = 0;
+    for (int col = 0; col < n && r < rows; col++) {
+        int piv = -1;
+        for (int q = r; q < rows; q++)
+            if (!A[q][col].is_zero()) { piv = q; break; }
+        if (piv < 0) continue;
+        std::swap(A[piv], A[r]);
+        const Fe inv = F.inv(A[r][col]);
+        for (auto& e : A[r]) e = F.mul(e, inv);
+        for (int q = 0; q < rows; q++) {
+            if (q == r || A[q][col].is_zero()) continue;
+            const Fe m = A[q][col];
+            for (int i = 0; i <= n; i++) A[q][i] = F.sub(A[q][i], F.mul(m, A[r][i]));
+        }
+        pivcol.push_back(col);
+        r++;
+    }
+    for (int q = r; q < rows; q++)
+        if (!A[q][n].is_zero()) return false;
+    c.assign((size_t)n, F.zero());
+    for (int j = 0; j < r; j++) c[(size_t)pivcol[j]] = A[j][n];
+    k = f[0];
+    for (int i = 0; i < n; i++) k = F.sub(k, F.mul(c[i], g[i][0]));
+    return true;
+}
+
+// The partial rounds of a t = 3 sparse schedule as a recurrence on lane 0 alone.  Lanes 1, 2 form a linear system driven by
+// the S-box outputs, so by Cayley-Hamilton on its 2x2 matrix B (z^2 + d1 z + d2) the lane-0 value x_k+1 after the constant
+// addition of round k+1 is, for k >= 2,
+//     x_k+1 = m00 y_k + b1 y_k-1 + b2 y_k-2 - d1 x_k - d2 x_k-1 + c_k,      y_k = x_k^alpha,
+// with the same five coefficients in every round and c_k fixed by the round constants.  Rounds 0 and 1 get rows of their own over
+// the lanes still held on entry (round 0: (y_0, s1, s2, x_0, 0); round 1: (y_1, y_0, s1, x_1, x_0), s2 eliminated through x_1), and
+// after the last round lanes 1, 2 are affine in (y_rp-1, y_rp-2, lane 0, x_rp-1).  Every coefficient is solved for exactly on
+// affine forms of the sparse rounds (sp, pc), so the kernels reproduce the sparse state bit for bit; false when a system has no
+// solution (e.g. w_hat[2] of round 0 is zero, or the last two lane-0 values do not determine lanes 1, 2).
+inline bool derive_recurrence(const Field& F, int rp, const FeVec& sp, const FeVec& pc, FeVec& rows, FeVec& ck, FeVec& rr) {
+    const int w = 5, nv = 4 + rp;
+    if (rp < 3) return false;                      // two bootstrap rounds, then at least one recurrence round
+    auto var = [&](int v) { return form_var(F, nv, v); };
+    FeVec l1 = var(1), l2 = var(2);
+    std::vector<FeVec> x{var(3)};                 // x[k]: lane 0 after the constant addition of round k; x[rp]: after the last round
+    for (int k = 0; k < rp; k++) {
+        const Fe* row = &sp[(size_t)k * w];
+        const FeVec y = var(4 + k);
+        FeVec d((size_t)nv, F.zero());
+        form_axpy(F, d, row[0], y);
+        form_axpy(F, d, row[1], l1);
+        form_axpy(F, d, row[2], l2);
+        form_axpy(F, l1, row[3], y);
+        form_axpy(F, l2, row[4], y);
+        if (k + 1 < rp) d[0] = F.add(d[0], pc[(size_t)k + 1]);
+        x.push_back(d);
+    }
+    rows.clear(); ck.clear(); rr.clear();
+    for (int k = 0; k < rp; k++) {
+        const std::vector<FeVec> h{var(4 + k), var(k >= 1 ? 3 + k : 1), var(k >= 2 ? 2 + k : k == 1 ? 1 : 2), x[(size_t)k],
+                                   k >= 1 ? x[(size_t)k - 1] : var(-1)};
+        FeVec c;
+        Fe c0;
+        if (!solve_affine(F, x[(size_t)k + 1], h, c, c0)) return false;
+        if (k <= 2) rows.insert(rows.end(), c.begin(), c.end());
+        else if (!std::equal(c.begin(), c.end(), rows.begin() + 2 * w)) return false;
+        ck.push_back(c0);
+    }
+    const std::vector<FeVec> h{var(3 + rp), var(2 + rp), x[(size_t)rp], x[(size_t)rp - 1]};
+    FeVec c1, c2;
+    Fe k1, k2;
+    if (!solve_affine(F, l1, h, c1, k1) || !solve_affine(F, l2, h, c2, k2)) return false;
+    rr = c1;
+    rr.insert(rr.end(), c2.begin(), c2.end());
+    rr.push_back(k1);
+    rr.push_back(k2);
     return true;
 }
 }  // namespace detail
@@ -287,8 +390,25 @@ inline PoseidonSchedule derive_schedule(const Field& F, const PoseidonParams& P,
         }
         S.off_sc0 = push(FeVec(1, y));
     }
+    FeVec rrows, rk, rr;
+    if (sparse && t == 3 && detail::derive_recurrence(F, rp, sp, pc, rrows, rk, rr)) {
+        S.recur = 1;
+        S.off_rc = push(rrows);
+        S.off_rk = push(rk);
+        S.off_rr = push(rr);
+    }
     S.n_elems = (int)(S.consts.size() / 4);
     return S;
+}
+
+// The kernels' view of a schedule.
+inline PoseidonDev make_dev(const PoseidonSchedule& S) {
+    PoseidonDev D;
+    D.t = S.t; D.rate = S.rate; D.cap = S.capacity; D.rf = S.rf; D.rp = S.rp; D.sparse = S.sparse; D.alpha = S.alpha;
+    D.off_c = S.off_c; D.off_m = S.off_m; D.off_mpre = S.off_mpre; D.off_cp0 = S.off_cp0; D.off_pc = S.off_pc;
+    D.off_sp = S.off_sp; D.off_arkp = S.off_arkp; D.off_mod = S.off_mod; D.off_sc0 = S.off_sc0; D.n_elems = S.n_elems; D.zero = 0;
+    D.recur = S.recur; D.off_rc = S.off_rc; D.off_rk = S.off_rk; D.off_rr = S.off_rr;
+    return D;
 }
 
 }  // namespace host
